@@ -8,6 +8,7 @@ reference's default wall geometry for that box (geodesic -> line_of_sight,
 ratinabox/Neurons.py:922-928), dt = 10 ms, history + spikes on (reference defaults).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c2e|c3|c4]
+                  [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); agents are sharded (weak scaling:
 65 536 agents per GPU), there is no collective on the step path.
@@ -270,10 +271,40 @@ def algorithmic_bytes_per_agent_step(n_cells, spikes):
     return 2 * 12 * 8 + 8 * 4 + 4 * n_cells + (n_cells // 8 if spikes else 0)
 
 
+DUMP_BYTES = 60_000_000           # all arrays together, .npy headers aside: under 64 MB
+DUMP_STATE = ("pos", "velocity", "rotational_velocity", "measured_velocity", "measured_rotational_velocity", "head_direction",
+              "distance_travelled", "distance_to_closest_wall")
+
+
+def dump_outputs(out_dir, Ag, pops, spikes):
+    """What a caller of Agent.run() receives after its last step, as <out_dir>/<name>.npy: the Agent's state (float64) and,
+    per population k, that step's firing rates (rates_<k>, float32) and spikes (spikes_<k>, 0 / 1 as float32).  Arrays of
+    every agent while they fit in DUMP_BYTES, else the rows of a fixed seeded sample of agents (agent_rows.npy)."""
+    import torch
+    from ratinabox_b200.Neurons import _unpack_spikes
+    os.makedirs(out_dir, exist_ok=True)
+    A = Ag.n_agents
+    state = {name: Ag.state_view(name) for name in DUMP_STATE}          # (A, ...) float64, read-only views
+    per_agent = 8 * (1 + sum(v[0].size for v in state.values())) + 4 * sum(ns.n for ns in pops) * (2 if spikes else 1)
+    n_rows = min(A, DUMP_BYTES // per_agent)
+    rows = np.arange(A) if n_rows == A else np.sort(np.random.default_rng(0).choice(A, n_rows, replace=False))
+    idx = torch.as_tensor(rows, device=Ag.device)
+    out = {"agent_rows": rows.astype(np.float64)}
+    for name, v in state.items():
+        out[name] = np.array(v[rows], dtype=np.float64)
+    for k, ns in enumerate(pops):
+        out[f"rates_{k}"] = ns._hist[ns._last_slot][idx, : ns.n].cpu().numpy()
+        if spikes:
+            out[f"spikes_{k}"] = _unpack_spikes(ns._spk[ns._last_slot][idx].cpu().numpy(), ns.n).astype(np.float32)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), arr)
+
+
 def measure(rb, lib, torch, dist, name, steps, warmup, rank, world, local_rank, spikes=True, total_agents=None, e2e=True,
-            keep=False):
+            keep=False, dump=None):
     """Device-resident throughput (riab_run, CUDA events, max over ranks) and the stepped-API e2e number of one workload.
-    total_agents: strong-scaling variant (that many agents in total, split over the ranks)."""
+    total_agents: strong-scaling variant (that many agents in total, split over the ranks).  dump: directory that receives
+    rank 0's outputs of the last timed step (dump_outputs)."""
     wl = WORKLOADS[name]
     if total_agents is not None:
         A, scaling = total_agents // world, "strong"
@@ -318,6 +349,8 @@ def measure(rb, lib, torch, dist, name, steps, warmup, rank, world, local_rank, 
     barrier()
     launches = lib.riab_launch_count() - l0
     ms = max_over_ranks(ev0.elapsed_time(ev1))
+    if dump is not None and rank == 0:
+        dump_outputs(dump, Ag, pops, spikes)
     res = {"agents_per_gpu": A, "agents_total": A * world, "n_cells": n_cells, "scaling": scaling, "steps": steps,
            "ms_per_step": ms / steps, "value": world * A * steps / (ms * 1e-3), "gpu_launches": int(launches)}
     bytes_unit = algorithmic_bytes_per_agent_step(n_cells, spikes)
@@ -440,7 +473,11 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the `workloads` / `strong` / `gather` objects")
     ap.add_argument("--agents", type=int, default=None,
                     help="experiments only: agents per GPU instead of the workload's (the line's config says so)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed run computed in its last step to DIR/<name>.npy (agent state, rates, spikes)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.agents is not None:                          # experiment: same workload at another batch size
         w0 = WORKLOADS[args.workload]
         WORKLOADS[args.workload] = dict(w0, agents=args.agents, desc=w0["desc"] + f" [--agents {args.agents}: NOT the configuration]")
@@ -483,7 +520,7 @@ def main():
     sampler = ClockSampler(local_rank)
     sampler.start()
     head = measure(rb, lib, torch, dist, args.workload, args.steps, args.warmup, rank, world, local_rank, spikes=spikes,
-                   keep=(world > 1 and not args.no_extra))
+                   keep=(world > 1 and not args.no_extra), dump=args.dump_outputs)
     clocks = sampler.stop()        # sampled across the device-resident and the e2e timed regions of the headline workload
     peaks = {}
     try:

@@ -13,6 +13,8 @@ Fixtures
                      (SURVEY.md section 8c mode A): inputs, outputs, collision masks.
   modeA_rates.npz    get_state(evaluate_at=None, pos=P) for every cell type/variant,
                      zero jitter.
+  host_mirror.npz    Environment / utils set-up helpers under fixed np.random seeds.
+  config1.npz        config 1 teacher-forced for 300 steps, open box and box + 2 walls.
 """
 import contextlib
 import os
@@ -39,9 +41,9 @@ def maze_walls(n=8, length=0.6):
 
 
 @contextlib.contextmanager
-def mode_a(tape):
+def mode_a(tape, used=None):
     """Zero the geometry jitter and feed ``scale == dt`` normals from ``tape``
-    (a list that is popped from the front)."""
+    (a list that is popped from the front); the standard normals drawn are appended to ``used``."""
     orig = np.random.normal
 
     def patched(loc=0.0, scale=1.0, size=None):
@@ -49,6 +51,8 @@ def mode_a(tape):
             return np.zeros(size)
         n = int(np.prod(size)) if size not in (None, ()) else 1
         vals = np.array([tape.pop(0) if tape else 0.0 for _ in range(n)], dtype=float)
+        if used is not None:
+            used.extend(vals.tolist())
         out = loc + scale * vals
         return out.reshape(size) if size not in (None, ()) else float(out[0])
 
@@ -199,7 +203,7 @@ def main():
 
     # ---------------------------------------------------------- modeA_rates
     rs = np.random.RandomState(4321)
-    P = rs.uniform(0.001, 0.999, size=(384, 2))
+    P = rs.uniform(0.001, 0.999, size=(384, 2))[:160]       # the first 160 of 384 draws keep the fixture under 1 MB
     res = {"P": P}
     with mode_a([]):
         Env = Environment()
@@ -606,6 +610,68 @@ def gen_host_utils():
     print("host_utils.npz", {k: v.shape for k, v in out.items() if k.startswith("assembly")})
 
 
+def gen_host_mirror():
+    """The 2 x 1 box with a doorway (Environment walls, extent, discretisation, sample_positions under np.random.seed(5))
+    and the set-up helpers (distribution_sampler, create_random_assembly, rotate) that the host mirror must reproduce bit
+    for bit -> tests/golden/host_mirror.npz."""
+    riab = ref_shim.import_reference()
+    assert riab is not None, "reference not present"
+    from ratinabox.Environment import Environment
+    from ratinabox import utils
+    R = Environment({"aspect": 2, "scale": 1})
+    R.add_wall([[1, 0], [1, 0.35]])
+    R.add_wall([[1, 0.65], [1, 1]])
+    out = {"walls": R.walls, "extent": np.asarray(R.extent, dtype=float), "flattened_discrete_coords": R.flattened_discrete_coords}
+    for method, n in (("uniform_jitter", 100), ("uniform", 30), ("random", 7), ("uniform_jitter", 1024)):
+        np.random.seed(5)
+        out[f"sample_{method}_{n}"] = R.sample_positions(n=n, method=method)
+    for name, prm, shape in (("uniform", (0.2, 1.0), (9,)), ("modules", (0.3, 0.5, 0.8), (10,)), ("rayleigh", (0.3,), (5,)),
+                             ("normal", (0, 1), (4, 2)), ("logarithmic", (0.1, 1.0), (6,)), ("delta", (0.4,), (3,))):
+        np.random.seed(3)
+        out[f"dist_{name}"] = np.asarray(utils.distribution_sampler(name, prm, shape))
+    np.random.seed(4)
+    out["assembly_n12"] = np.stack(utils.create_random_assembly(n=12))
+    out["rotate"] = utils.rotate(np.array([1, 0]), 0.3)
+    np.savez_compressed(os.path.join(GOLD, "host_mirror.npz"), **out)
+    print("host_mirror.npz", {k: v.shape for k, v in out.items()})
+
+
+def gen_config1():
+    """BASELINE.json configs[0] (1 agent, default box, 100 Gaussian PlaceCells, dt = 10 ms) in the open box and with the
+    two internal walls, 300 steps of the reference teacher-forced like mode A: geometry jitter zeroed, the `scale == dt`
+    normals fed from RandomState(7).  Per step the Agent's state before it, the two Ornstein-Uhlenbeck normals it drew and
+    the firing rates after it -> tests/golden/config1.npz."""
+    import ref_driver
+    steps, N = 300, 100
+    state = ("pos", "velocity", "rotational_velocity", "measured_velocity", "head_direction", "distance_travelled")
+    out = {}
+    for name, walls in (("open", []), ("box2", BOX_WALLS)):
+        rs = np.random.RandomState(7)
+        centres = rs.uniform(0.05, 0.95, (N, 2))
+        geom = "line_of_sight" if walls else "euclidean"
+        _, _, RA, (RP,) = ref_driver.build(walls, [("place", {"n": N, "place_cell_centres": centres, "widths": 0.2,
+                                                              "wall_geometry": geom}, None)],
+                                           pos=[0.5, 0.52], vel=[0.05, 0.06], dt=0.01, seed=3)
+        rec = {k: [np.array(getattr(RA, k), dtype=float)] for k in state}
+        xi, fr = [], []
+        for s in range(steps):
+            tape, used = rs.normal(size=2 + N).tolist(), []
+            with mode_a(tape, used):
+                RA.update()
+                RP.update()
+            assert len(used) <= 2 + N                       # every draw came from the tape
+            xi.append(used[:2])
+            fr.append(np.array(RP.firingrate, dtype=float))
+            for k in state:
+                rec[k].append(np.array(getattr(RA, k), dtype=float))
+        out[f"{name}_walls"] = np.array(walls, dtype=float).reshape(-1, 2, 2)
+        out[f"{name}_centres"], out[f"{name}_xi"], out[f"{name}_rates"] = centres, np.array(xi), np.array(fr)
+        for k in state:
+            out[f"{name}_{k}"] = np.array(rec[k])
+    np.savez_compressed(os.path.join(GOLD, "config1.npz"), **out)
+    print("config1.npz", os.path.getsize(os.path.join(GOLD, "config1.npz")) // 1024, "KiB")
+
+
 if __name__ == "__main__":
     if sys.argv[1:] == ["api"]:
         gen_api_defaults()
@@ -619,6 +685,10 @@ if __name__ == "__main__":
         gen_polygon()
     elif sys.argv[1:] == ["ovc"]:
         gen_ovc()
+    elif sys.argv[1:] == ["mirror"]:
+        gen_host_mirror()
+    elif sys.argv[1:] == ["config1"]:
+        gen_config1()
     else:
         main()
         gen_polygon()
@@ -627,3 +697,5 @@ if __name__ == "__main__":
         gen_histogram()
         gen_api_defaults()
         gen_host_utils()
+        gen_host_mirror()
+        gen_config1()

@@ -6,7 +6,7 @@ Stages the UNMODIFIED reference package so that it can travel to the GPU box:
 
 `oracle/_ref/` is git-ignored (reference sources never enter this repository's history) but NOT gpurun-ignored, exactly
 like the built `.so`: `bench.py --impl reference`, `bench.py`'s `cpu_baseline` leg and
-`tests/test_gpu_vs_reference.py` import the live reference from there through `oracle/ref_shim.py` (stand-ins for the
+`tests/test_gpu_reference_binding.py` import the live reference from there through `oracle/ref_shim.py` (stand-ins for the
 absent matplotlib / shapely).  Only Python sources are staged (the 7 MB of trajectory datasets under `ratinabox/data` are
 not on the hot path); files are copied byte for byte and a manifest with their SHA-256 is written next to them.
 `__graft_entry__.build()` runs this whenever /root/reference is present."""

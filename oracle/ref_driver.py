@@ -1,6 +1,6 @@
 """TEST / BASELINE INFRASTRUCTURE -- drives the UNMODIFIED reference (ratinabox v1.15.3) the way its users do:
 one Agent per Python object, `Ag.update(); Ns.update()` in a Python loop (tests/test_advanced.py:17-23 of the reference).
-Used by bench.py's CPU legs (`--impl reference`, `cpu_baseline`) and tests/test_gpu_vs_reference.py; never by the product."""
+Used by bench.py's CPU legs (`--impl reference`, `cpu_baseline`) and oracle/gen_golden.py config1; never by the product."""
 import os
 import sys
 

@@ -3,7 +3,7 @@
 Used by ``oracle/gen_golden.py`` (build container, /root/reference) to pin the
 oracle restatement against the live reference, and -- through the copy that
 ``oracle/make_ref.py`` stages into the git-ignored ``oracle/_ref/`` -- by
-``bench.py``'s CPU legs and ``tests/test_gpu_vs_reference.py`` on the GPU box.
+``bench.py``'s CPU legs and ``tests/test_gpu_reference_binding.py`` on the GPU box.
 Nothing in the product path imports this file.
 
 The reference imports matplotlib and shapely at module top

@@ -29,6 +29,15 @@ def _f64p(a):
     return a.ctypes.data_as(_lib.c_double_p)
 
 
+def _unpack_spikes(words, n):
+    """Spike words (..., W) int32 of the device rings -> (..., n) bool."""
+    lead = words.shape[:-1]
+    bits = np.unpackbits(words.view(np.uint8), axis=-1, bitorder="little")
+    # bit L of word 4B+i = cell 128B + 4L + i  (one warp ballot per cell slot i)
+    bits = bits.reshape(*lead, -1, 4, 32).swapaxes(-1, -2).reshape(*lead, -1)
+    return bits[..., :n].astype(bool)
+
+
 class Neurons:
     default_params = {                                              # ratinabox/Neurons.py:90-99
         "n": 10,
@@ -266,11 +275,7 @@ class Neurons:
                 start = self._hist_rows % self._hist_cap if self._hist_rows > self._hist_cap else 0
                 idx = (torch.arange(n, device=self.device) + start) % self._hist_cap
                 fr = self._hist[idx][:, :, : self.n].cpu().numpy().astype(np.float64)
-                words = self._spk[idx].cpu().numpy().view(np.uint32)
-                # bit L of word 4B+i = cell 128B + 4L + i  (one warp ballot per cell slot i)
-                bits = np.unpackbits(words.view(np.uint8), axis=-1, bitorder="little")
-                bits = bits.reshape(n, A, -1, 4, 32).transpose(0, 1, 2, 4, 3).reshape(n, A, -1)
-                sp = bits[:, :, : self.n].astype(bool)
+                sp = _unpack_spikes(self._spk[idx].cpu().numpy(), self.n)
             if A == 1:
                 fr, sp = fr[:, 0], sp[:, 0]
             self.history_dropped = self._hist_rows - n

@@ -1,6 +1,6 @@
 """CPU-only checks: the C-ABI library loads and exports every symbol include/riab_b200.h
 declares; the host-side packers agree with NumPy; the host mirror of Environment agrees
-with the oracle (and with the live reference when it is present); sharding helpers work
+with the oracle and with the reference's stored outputs (tests/golden); sharding helpers work
 under a world_size-2 gloo group.  No CUDA calls."""
 import ctypes as C
 import os
@@ -125,7 +125,8 @@ def test_grid_and_bvc_pack():
     assert lib.riab_bvc_scratch_floats(33, T) == 2 * T * 32
 
 
-def test_environment_mirror_matches_oracle_and_reference():
+def test_environment_mirror_matches_oracle_and_reference(golden):
+    """The reference's side is tests/golden/host_mirror.npz (oracle/gen_golden.py mirror)."""
     import ratinabox_b200 as rb
     E = rb.Environment({"aspect": 2, "scale": 1})
     E.add_wall([[1, 0], [1, 0.35]])
@@ -133,37 +134,27 @@ def test_environment_mirror_matches_oracle_and_reference():
     env = O.OracleEnvironment(scale=1, aspect=2, walls=[[[1, 0], [1, 0.35]], [[1, 0.65], [1, 1]]])
     assert np.array_equal(E.walls, env.walls) and np.array_equal(E.extent, env.extent)
     assert E.check_if_position_is_in_environment([0.5, 0.5]) and not E.check_if_position_is_in_environment([2.0, 0.5])
-    import ref_shim
-    if ref_shim.import_reference() is None:
-        pytest.skip("live reference not present (GPU box)")
-    from ratinabox.Environment import Environment as RefEnv
-    R = RefEnv({"aspect": 2, "scale": 1})
-    R.add_wall([[1, 0], [1, 0.35]])
-    R.add_wall([[1, 0.65], [1, 1]])
-    assert np.array_equal(R.walls, E.walls) and np.array_equal(R.extent, E.extent)
-    assert np.array_equal(R.flattened_discrete_coords, E.flattened_discrete_coords)
+    R = golden("host_mirror.npz")
+    assert np.array_equal(R["walls"], E.walls) and np.array_equal(R["extent"], E.extent)
+    assert np.array_equal(R["flattened_discrete_coords"], E.flattened_discrete_coords)
     for method, n in (("uniform_jitter", 100), ("uniform", 30), ("random", 7), ("uniform_jitter", 1024)):
-        np.random.seed(5); a = R.sample_positions(n=n, method=method)
         np.random.seed(5); b = E.sample_positions(n=n, method=method)
-        assert np.array_equal(a, b), method
+        assert np.array_equal(R[f"sample_{method}_{n}"], b), method
 
 
-def test_set_up_helpers_match_reference():
-    import ref_shim
-    if ref_shim.import_reference() is None:
-        pytest.skip("live reference not present (GPU box)")
-    from ratinabox import utils as RU
+def test_set_up_helpers_match_reference(golden):
+    """The reference's side is tests/golden/host_mirror.npz (oracle/gen_golden.py mirror)."""
     from ratinabox_b200 import utils as U
+    R = golden("host_mirror.npz")
     for name, prm, shape in (("uniform", (0.2, 1.0), (9,)), ("modules", (0.3, 0.5, 0.8), (10,)), ("rayleigh", (0.3,), (5,)),
                              ("normal", (0, 1), (4, 2)), ("logarithmic", (0.1, 1.0), (6,)), ("delta", (0.4,), (3,))):
-        np.random.seed(3); a = RU.distribution_sampler(name, prm, shape)
         np.random.seed(3); b = U.distribution_sampler(name, prm, shape)
-        assert np.array_equal(a, b), name
-    np.random.seed(4); a = RU.create_random_assembly(n=12)
+        assert np.array_equal(R[f"dist_{name}"], b), name
     np.random.seed(4); b = U.create_random_assembly(n=12)
-    for x, y in zip(a, b):
+    assert len(b) == len(R["assembly_n12"])
+    for x, y in zip(R["assembly_n12"], b):
         assert np.array_equal(x, y)
-    assert np.array_equal(RU.rotate(np.array([1, 0]), 0.3), U.rotate(np.array([1, 0]), 0.3))
+    assert np.array_equal(R["rotate"], U.rotate(np.array([1, 0]), 0.3))
 
 
 def test_product_path_never_imports_the_oracle():

@@ -1,6 +1,7 @@
 """INTEGRATION.md section 2 as a test: subclasses of the REFERENCE's own Agent / PlaceCells (examples/reference_binding.py)
 whose update() / get_state() call the C ABI, run next to the unmodified classes on the same taped normals.  GPU only;
 skipped when the reference is not importable (oracle/_ref not staged)."""
+import contextlib
 import os
 import sys
 
@@ -11,8 +12,29 @@ pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
-sys.path.insert(0, os.path.join(ROOT, "tests"))
 import ref_driver  # noqa: E402
+
+
+@contextlib.contextmanager
+def taped_normals(tape, used):
+    """np.random.normal as the reference calls it: jitter scales -> zeros, `scale == dt` draws -> popped from `tape`
+    (standard normals; the reference scales them itself) and logged in `used`."""
+    orig = np.random.normal
+
+    def patched(loc=0.0, scale=1.0, size=None):
+        if scale in (1e-9, 1e-6):
+            return np.zeros(size)
+        n = int(np.prod(size)) if size not in (None, ()) else 1
+        vals = np.array([tape.pop(0) for _ in range(n)], dtype=float)
+        used.extend(vals.tolist())
+        out = loc + scale * vals
+        return out.reshape(size) if size not in (None, ()) else float(out[0])
+
+    np.random.normal = patched
+    try:
+        yield
+    finally:
+        np.random.normal = orig
 
 
 @pytest.mark.skipif(not ref_driver.available(), reason="oracle/_ref not staged (python oracle/make_ref.py)")
@@ -20,7 +42,6 @@ def test_reference_classes_step_on_the_gpu_through_the_c_abi():
     import ref_shim
     ref_shim.import_reference()
     sys.path.insert(0, os.path.join(ROOT, "examples"))
-    from test_gpu_vs_reference import taped_normals
     import reference_binding as B
     from ratinabox.Environment import Environment
     from ratinabox.Agent import Agent

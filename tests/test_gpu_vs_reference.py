@@ -1,55 +1,26 @@
-"""The CUDA path against the LIVE, unmodified reference (RatInABox v1.15.3 staged in oracle/_ref by oracle/make_ref.py,
-imported through oracle/ref_shim.py) -- no oracle restatement in between.  BASELINE.json configs[0]: 1 agent, default box,
-100 Gaussian PlaceCells, dt = 10 ms.  Teacher-forced like the oracle's mode A: the reference's geometry jitter is zeroed and
-its `scale == dt` normals are taped, every step starts from the reference's state.  Skipped when the staged reference is
-absent (run `python oracle/make_ref.py` in the build container; gpurun ships oracle/_ref like the built .so).  GPU only."""
-import contextlib
-import os
-import sys
-
+"""The CUDA path against the unmodified reference (RatInABox v1.15.3) -- no oracle restatement in between.  BASELINE.json
+configs[0]: 1 agent, default box, 100 Gaussian PlaceCells, dt = 10 ms.  Teacher-forced like the oracle's mode A: the
+reference's geometry jitter is zeroed and its `scale == dt` normals are taped, every step starts from the reference's state.
+The reference's 300 steps are stored in tests/golden/config1.npz (oracle/gen_golden.py config1).  GPU only."""
 import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "oracle"))
-import ref_driver  # noqa: E402
+STATE = ("pos", "velocity", "rotational_velocity", "measured_velocity", "head_direction", "distance_travelled")
 
 
-@contextlib.contextmanager
-def taped_normals(tape, used):
-    """np.random.normal as the reference calls it: jitter scales -> zeros, `scale == dt` draws -> popped from `tape`
-    (standard normals; the reference scales them itself) and logged in `used`."""
-    orig = np.random.normal
-
-    def patched(loc=0.0, scale=1.0, size=None):
-        if scale in (1e-9, 1e-6):
-            return np.zeros(size)
-        n = int(np.prod(size)) if size not in (None, ()) else 1
-        vals = np.array([tape.pop(0) for _ in range(n)], dtype=float)
-        used.extend(vals.tolist())
-        out = loc + scale * vals
-        return out.reshape(size) if size not in (None, ()) else float(out[0])
-
-    np.random.normal = patched
-    try:
-        yield
-    finally:
-        np.random.normal = orig
-
-
-@pytest.mark.skipif(not ref_driver.available(), reason="oracle/_ref not staged (python oracle/make_ref.py)")
 @pytest.mark.parametrize("walls", [[], [[[0.3, 0.0], [0.3, 0.5]], [[0.7, 1.0], [0.7, 0.5]]]])
-def test_config1_against_the_live_reference(walls):
+def test_config1_against_the_live_reference(golden, walls):
     import ratinabox_b200 as rb
-    steps, N = 300, 100
-    rs = np.random.RandomState(7)
-    centres = rs.uniform(0.05, 0.95, (N, 2))
+    g = golden("config1.npz")
+    name = "box2" if walls else "open"
+    assert np.array_equal(g[f"{name}_walls"], np.array(walls, dtype=float).reshape(-1, 2, 2))
+    centres, xi, ref_rates = g[f"{name}_centres"], g[f"{name}_xi"], g[f"{name}_rates"]
+    ref_state = {k: g[f"{name}_{k}"] for k in STATE}
+    steps, N = len(xi), len(centres)
+    assert steps == 300 and N == 100
     geom = "line_of_sight" if walls else "euclidean"
-    _, _, RA, (RP,) = ref_driver.build(walls, [("place", {"n": N, "place_cell_centres": centres, "widths": 0.2,
-                                                          "wall_geometry": geom}, None)],
-                                       pos=[0.5, 0.52], vel=[0.05, 0.06], dt=0.01, seed=3)
     np.random.seed(5)
     E = rb.Environment()
     for w in walls:
@@ -57,18 +28,12 @@ def test_config1_against_the_live_reference(walls):
     Ag = rb.Agent(E, {"dt": 0.01})
     PCs = rb.PlaceCells(Ag, {"n": N, "place_cell_centres": centres, "widths": 0.2, "wall_geometry": geom})
     worst_p = worst_r = 0.0
-    state = ("pos", "velocity", "rotational_velocity", "measured_velocity", "head_direction", "distance_travelled")
     for s in range(steps):
-        for k in state:                                        # teacher forcing: start from the reference's state
-            setattr(Ag, k, np.array(getattr(RA, k), dtype=float))
-        tape, used = rs.normal(size=2 + N).tolist(), []
-        with taped_normals(tape, used):
-            RA.update()
-            RP.update()
-        Ag.update(_xi=np.array(used[:2]))                      # the reference's two OU draws of this step
+        for k in STATE:                                        # teacher forcing: start from the reference's state
+            setattr(Ag, k, np.array(ref_state[k][s], dtype=float))
+        Ag.update(_xi=xi[s])                                   # the reference's two OU draws of this step
         PCs.update()
-        worst_p = max(worst_p, float(np.abs(np.asarray(Ag.pos) - RA.pos).max()))
-        ref_fr = np.asarray(RP.firingrate, dtype=float)
-        worst_r = max(worst_r, float(np.abs(np.asarray(PCs.firingrate) - ref_fr).max()))
+        worst_p = max(worst_p, float(np.abs(np.asarray(Ag.pos) - ref_state["pos"][s + 1]).max()))
+        worst_r = max(worst_r, float(np.abs(np.asarray(PCs.firingrate) - ref_rates[s]).max()))
     assert worst_p <= 1e-6, worst_p                            # north_star: positions <= 1e-6 m
     assert worst_r <= 1e-5, worst_r                            # rates <= 1e-5 of the rate scale (max_fr = 1)
